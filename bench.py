@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA engine)
   python bench.py --impl reference --steps K --warmup W    # reference arm: CPU oracle port
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 metric: walker.local-energies / second.  A "step" = one local-energy evaluation of every walker
 of the batch (Psiformer forward + forward-Laplacian + potentials, incl. the non-local ECP
@@ -120,6 +121,32 @@ TRAFFIC = {
                           'source': 'profiles/r02_ncu_trunk_f16_kernel_ts.csv'},
 }
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, per_walker, other):
+    """Write one step's outputs as ``out_dir/<name>.npy`` in float32 or float64, so that two builds run with the same
+    arguments can be compared array by array.  ``per_walker`` arrays share a leading walker axis; if everything together
+    would exceed 64 MiB, they are cut to a fixed, seeded sample of walkers and ``walker_index.npy`` names the walkers kept."""
+    def host(x):
+        x = x.detach().cpu().numpy() if torch.is_tensor(x) else np.asarray(x)
+        return x.astype(np.float64 if x.dtype == np.float64 else np.float32)
+
+    per_walker = {k: host(v) for k, v in per_walker.items()}
+    other = {k: host(v) for k, v in other.items()}
+    n = next(iter(per_walker.values())).shape[0]
+    walker_bytes = sum(v.nbytes for v in per_walker.values()) // n
+    budget = DUMP_LIMIT_BYTES - sum(v.nbytes for v in other.values())
+    if walker_bytes * n > budget:
+        keep = budget // (walker_bytes + 8)  # 8 bytes per walker for walker_index itself
+        idx = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        per_walker = {k: v[idx] for k, v in per_walker.items()}
+        other['walker_index'] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in {**per_walker, **other}.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), v)
+
+
 _ORACLE = {}
 
 
@@ -235,7 +262,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--gemm-backend', default='tcgen05', choices=['simt', 'tcgen05'])
     ap.add_argument('--equil-sweeps', type=int, default=None)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write what the last timed step computed (rank 0's walkers) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA engine; the reference arm keeps none')
     wl = WORKLOADS[a.workload]
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -322,6 +355,8 @@ def main():
         smp_state = dict(r=r.clone(), sign=sign0, log=log0, age=torch.zeros(B, dtype=torch.int32, device=dev),
                          tau=torch.tensor([0.5], dtype=tdt, device=dev))
 
+    last = {}  # what the most recent step() handed back, by reference: --dump-outputs copies it after the timed loop
+
     def step(seed, pcs_=None):
         pcs_ = pcs_ or pcs
         if n_sub:
@@ -334,12 +369,13 @@ def main():
         for st in range(n_states):
             E, stt = loc_ene(seed, params_all[st], pcs_[st])
             Es.append(E); sts.append(stt)
+        last.update(r=[p_.r for p_ in pcs_], E=Es, stats=sts)
         if n_states > 1:  # pairwise overlap penalty: every state's wave function on every state's walkers (loss/overlap.py:19-150)
             from deepqmc_b200.overlap import compute_mean_overlap, compute_psi_ratio
 
             pc_all = PhysicalConfiguration(R, torch.stack([p_.r for p_ in pcs_]), torch.zeros(n_states, B, device=dev))
             ratio, _ = compute_psi_ratio(ansatz, params_all, pc_all)
-            compute_mean_overlap(ratio)
+            last['overlap'] = compute_mean_overlap(ratio)
             E = torch.cat(Es)
             return parallel.energy_statistics(E, {k: torch.cat([s_[k] for s_ in sts]) for k in sts[0]}), E
         return parallel.energy_statistics(Es[0], sts[0]), Es[0]
@@ -368,6 +404,13 @@ def main():
     t_wall = time.perf_counter() - t_wall0
     launches = eng.launch_count - l0
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:  # before the e2e leg: the sampler state of lih_eval_step moves on in place
+        per_walker = {'walkers': torch.cat(last['r']), 'E_loc': torch.cat(last['E'])}
+        per_walker.update({k.replace('/', '_'): torch.cat([s_[k] for s_ in last['stats']]) for k in last['stats'][0]})
+        other = {'stat_' + k.replace('/', '_'): v for k, v in stats.items()}
+        if 'overlap' in last:
+            other.update(overlap_loss=last['overlap'][0], overlap=last['overlap'][1]['overlap/pairwise/mean'])
+        dump_outputs(a.dump_outputs, per_walker, other)
     per_step = [e0.elapsed_time(e1) for e0, e1 in evs]
     ms = torch.tensor([sum(per_step)], device=dev, dtype=torch.float64)
     if world > 1:
@@ -384,9 +427,9 @@ def main():
         _, E = step(seed, pcs_h)
         return E.cpu()
     # long steps (seconds): the pipeline is warm already, bound the e2e leg to a few steps
-    # (same number of steps as the device-timed leg unless that would take more than ~2 minutes)
+    # (same number of steps as the device-timed leg unless that would take more than ~2 minutes; never more than --steps)
     slow = total_ms / a.steps > 500.0
-    e2e_warm, e2e_steps = (1, max(3, min(a.steps, int(120e3 / (total_ms / a.steps))))) if slow else (3, a.steps)
+    e2e_warm, e2e_steps = (1, min(a.steps, max(3, int(120e3 / (total_ms / a.steps))))) if slow else (3, a.steps)
     for w in range(e2e_warm):
         e2e_step(w)
     torch.cuda.synchronize()

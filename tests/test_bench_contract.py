@@ -22,6 +22,32 @@ def test_reference_arm_prints_the_contract_line():
     assert 'workload' in d['config'] and d['data'] == 'synthetic' and d['dtype'] == 'f64'
 
 
+def test_dump_outputs_writes_float_arrays_and_samples_walkers_over_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    import bench
+
+    per_walker = {'E_loc': torch.arange(100, dtype=torch.float32), 'walkers': torch.zeros(100, 4, 3, dtype=torch.float64),
+                  'hamil_V_el': torch.ones(100, dtype=torch.float32)}
+    other = {'stat_energy_count': torch.tensor(100.0, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / 'all'), per_walker, other)
+    e = np.load(tmp_path / 'all' / 'E_loc.npy')
+    assert e.dtype == np.float32 and np.array_equal(e, np.arange(100)) and not (tmp_path / 'all' / 'walker_index.npy').exists()
+    assert np.load(tmp_path / 'all' / 'walkers.npy').dtype == np.float64 and np.load(tmp_path / 'all' / 'stat_energy_count.npy') == 100
+
+    monkeypatch.setattr(bench, 'DUMP_LIMIT_BYTES', 4000)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), per_walker, other)
+    files = sorted(os.listdir(tmp_path / 'a'))
+    assert files == ['E_loc.npy', 'hamil_V_el.npy', 'stat_energy_count.npy', 'walker_index.npy', 'walkers.npy']
+    assert sum(np.load(tmp_path / 'a' / f).nbytes for f in files) <= 4000
+    idx = np.load(tmp_path / 'a' / 'walker_index.npy')
+    assert 0 < len(idx) < 100 and np.array_equal(np.load(tmp_path / 'a' / 'E_loc.npy'), idx)
+    for f in files:  # the sample is fixed: the same walkers every time
+        assert np.array_equal(np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f))
+
+
 def test_other_ranks_of_the_reference_arm_exit_quietly():
     env = dict(os.environ, RANK='1', WORLD_SIZE='2')
     cp = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--gpus', '2', '--workload',
